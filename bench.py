@@ -13,7 +13,9 @@ A "step" is one pass of the hot path over one batch of synthetic input, through 
 `roofline`= the observation-render kernel: algorithmic bytes per launch / mean launch duration (CUDA events
             around every launch inside the timed region) against the measured HBM copy bandwidth.
 `cpu_baseline` / `--impl reference` = the UNMODIFIED reference C++ engine (oracle/_ref/libmagent.so, built
-            from /root/reference by oracle/Makefile) driven by the same host code on this box's host cores.
+            by oracle/Makefile where the reference sources exist) driven by the same host code on the host cores;
+            without it, the plain-C restatement (oracle/_build), reported as `cpu_baseline.kind` = "port".
+`--dump-outputs DIR` writes what the device-resident loop computed in its last timed step (see dump_outputs).
 
 Workloads (BASELINE.json configs; the default is the per-GPU share of configs[4], weak scaling):
     battle512  battle 200x200, 2x1000 agents, 512 independent arenas per GPU          [default]
@@ -342,6 +344,30 @@ def make_clock_sampler(index, pci_bus_id=None):
     return ClockSampler(pci_bus_id or index)
 
 
+DUMP_BYTES = 64 * 10 ** 6 - 64 * 1024      # 64 MB with room for the .npy headers
+
+
+def dump_outputs(out_dir, bufs, nums, done, prefix=""):
+    """Write what the last timed step handed its caller, in float32: per acting group g the observation views
+    g<g>_view (n, H, W, C), the feature rows g<g>_feature (n, F) and the rewards g<g>_reward (n,) of the n agents it
+    observed, and the done flag.  Where that is more than 64 MB, every group keeps an equal share of its rows, drawn
+    with a fixed seed (g as the seed); g<g>_rows (float64) lists the rows kept."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // max(1, len(bufs))
+    for g, (v, f, r) in sorted(bufs.items()):
+        n = nums[g]
+        row_bytes = 4 * (int(np.prod(v.shape[1:])) + int(np.prod(f.shape[1:])) + 1) + 8
+        keep = min(n, budget // row_bytes)
+        rows = np.arange(n) if keep == n else np.sort(np.random.RandomState(g).choice(n, keep, replace=False))
+        idx = torch.from_numpy(rows).to(v.device)
+        for name, t in (("view", v), ("feature", f), ("reward", r)):
+            np.save(os.path.join(out_dir, "%sg%d_%s.npy" % (prefix, g, name)), t.index_select(0, idx).float().cpu().numpy())
+        np.save(os.path.join(out_dir, "%sg%d_rows.npy" % (prefix, g)), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, prefix + "done.npy"), done.float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -367,12 +393,16 @@ def main():
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="device-resident loop as a replayed CUDA graph of two steps (magent_b200_graph_*): auto = for "
                          "launch-bound workloads (fewer than 250k agents per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the observations, rewards and done flag of the last timed step to DIR/<name>.npy")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--_cpu-worker", dest="cpu_worker", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=100)
     ap.add_argument("--cpu-warmup", type=int, default=5)
     ap.add_argument("--cpu-seed", type=int, default=0)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.cpu_worker:
         return cpu_worker(args)
 
@@ -384,7 +414,8 @@ def main():
         for w in ("battle1", "gather64", "battle1m", "battle1m_sparse", "battle512"):
             cmd = [sys.executable, os.path.abspath(__file__), "--workload", w, "--steps", str(args.steps), "--warmup", str(args.warmup),
                    "--e2e-seconds", str(args.e2e_seconds)] + (["--no-cpu"] if args.no_cpu or w != "battle512" else []) + \
-                  (["--no-e2e"] if args.no_e2e else [])
+                  (["--no-e2e"] if args.no_e2e else []) + \
+                  (["--dump-outputs", os.path.join(args.dump_outputs, w)] if args.dump_outputs else [])
             r = subprocess.run(cmd, capture_output=True, text=True)
             sys.stdout.write(r.stdout if r.returncode == 0 else json.dumps({"workload": w, "failed": r.stderr[-400:]}) + "\n")
             sys.stdout.flush()
@@ -403,12 +434,15 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
+        if args.dump_outputs:
+            sys.exit("bench.py: --dump-outputs dumps the B200 arm's outputs; it does not apply to --impl reference")
         if not os.path.exists(REF_LIB):
-            # the reference arm is the UNMODIFIED reference or nothing: never silently the C restatement
-            sys.stderr.write("bench.py --impl reference: oracle/_ref/libmagent.so is missing (build it with "
-                             "`make -C oracle ref` where /root/reference exists)\n")
-            sys.exit(3)
+            # never silently the C restatement: the JSON line says cpu_baseline.kind = "port"
+            sys.stderr.write("bench.py --impl reference: oracle/_ref/libmagent.so is missing (`make -C oracle ref` builds it "
+                             "from the reference sources); timing the plain-C restatement instead\n")
         cb = run_cpu_baseline(args.workload, budget_steps=None)
+        if cb is None:
+            sys.exit("bench.py --impl reference: no CPU engine built (run __graft_entry__.build())")
         print(json.dumps({
             "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_sample_step"], "higher_is_better": True,
@@ -507,6 +541,13 @@ def main():
     use_graph = args.graph == "on" or (args.graph == "auto" and n_agents_now < 250000)
     graph_note = None
     steps_timed = args.steps
+    last_nums = {}
+
+    def last_step(s):
+        # the group sizes the last step observes; the engine settles them with a host wait, so only when dumping
+        if args.dump_outputs:
+            last_nums.update({env._hv(h): env.get_num(h) for h in act})
+        dev_step(s)
     barrier()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     if use_graph:
@@ -523,13 +564,18 @@ def main():
         l_cap = env.launch_count()
         gid = env.capture_graph(lambda: (dev_step(0), dev_step(1)))
         per_replay = env.launch_count() - l_cap
-        replays = max(1, args.steps // 2)
-        steps_timed = 2 * replays
+        # an odd last step (and, when dumping, the last step, whose group sizes are read first) runs un-captured
+        replays = (args.steps - 1) // 2 if args.dump_outputs else args.steps // 2
+        tail = args.steps - 2 * replays
         env.launch_graph(gid, 2)                        # warm the instantiated graph
         barrier()
         c0 = env.get_counters()
         ev0.record()
-        env.launch_graph(gid, replays)
+        if replays:
+            env.launch_graph(gid, replays)
+        l_tail = env.launch_count()
+        for s in range(tail):
+            (last_step if s == tail - 1 else dev_step)(2 * replays + s)
         ev1.record()
         if sampler:
             sampler.sample_now()                        # the host is ahead of the GPU here: a sample inside the timed region
@@ -537,15 +583,16 @@ def main():
         ms = ev0.elapsed_time(ev1)
         barrier()
         c1 = env.get_counters()
-        launches = per_replay * replays
-        graph_note = "CUDA graph of 2 steps (%d kernels) replayed %d times" % (per_replay, replays)
+        launches = per_replay * replays + env.launch_count() - l_tail
+        graph_note = "CUDA graph of 2 steps (%d kernels) replayed %d times" % (per_replay, replays) + \
+            (", then %d un-captured step(s)" % tail if tail else "")
     else:
         c0 = env.get_counters()
         l0 = env.launch_count()
         env.set_profiling(True)
         ev0.record()
         for s in range(args.steps):
-            dev_step(s)
+            (last_step if s == args.steps - 1 else dev_step)(s)
         ev1.record()
         if sampler:
             sampler.sample_now()                        # everything is queued, the GPU is mid-way: a sample inside the timed region
@@ -557,6 +604,8 @@ def main():
         c1 = env.get_counters()
         launches = env.launch_count() - l0
     agent_steps = c1[0] - c0[0]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bufs, last_nums, done_dev, "rank%d_" % rank if world > 1 else "")
 
     if os.environ.get("MAGENT_B200_BENCH_RANK_REPORT"):
         sys.stderr.write("rank %d: %.4f ms/step device time, render %.4f ms/launch, %d launches\n"

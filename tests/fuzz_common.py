@@ -180,14 +180,19 @@ def make_env(lib, seed, **kw):
     return env
 
 
-def play(seed, lib_a, lib_b, steps=25, **kw):
+def trace(seed, lib, steps=25, **kw):
+    """the random game of `seed` played on one engine library (pc.run_trace record list)"""
     rs = np.random.RandomState(seed)
-    n_groups = len(make_env(lib_a, seed).get_handles())
+    n_groups = len(make_env(lib, seed).get_handles())
     order = [int(g) for g in rs.permutation(n_groups)]
     acting = sorted(int(g) for g in rs.choice(n_groups, size=int(rs.randint(1, n_groups + 1)), replace=False))
     order = [g for g in order if g in acting]
-    a = pc.run_trace(make_env(lib_a, seed), steps, seed, keep_obs=True, act_groups=acting, order=order, stop_on_done=False)
-    b = pc.run_trace(make_env(lib_b, seed, **kw), steps, seed, keep_obs=True, act_groups=acting, order=order, stop_on_done=False)
+    return pc.run_trace(make_env(lib, seed, **kw), steps, seed, keep_obs=True, act_groups=acting, order=order, stop_on_done=False)
+
+
+def play(seed, lib_a, lib_b, steps=25, **kw):
+    a = trace(seed, lib_a, steps)
+    b = trace(seed, lib_b, steps, **kw)
     pc.compare_traces(a, b, what="fuzz seed %d" % seed)
     return a
 
@@ -413,21 +418,26 @@ def trace_chaotic(env, steps, seed, acting, order, render_dir=None):
         return e.value
 
 
-def play_chaotic(seed, lib_a, lib_b, steps=24, **kw):
+def chaotic_log(seed, lib, steps=24, **kw):
+    """the chaotic caller of `seed` on one engine library (trace_chaotic record list)"""
     rs = np.random.RandomState(seed)
-    n_groups = len(make_env(lib_a, seed).get_handles())
+    n_groups = len(make_env(lib, seed).get_handles())
     order = [int(g) for g in rs.permutation(n_groups)]
+    import shutil
     import tempfile
     # with more than 4 groups the reference indexes its 4-row colour table out of bounds (RenderGenerator.cc gen_config:
     # uninitialised stack in config.json)
-    can_render = n_groups <= 4
-    da, db = (tempfile.mkdtemp(), tempfile.mkdtemp()) if can_render else (None, None)
-    a = trace_chaotic(make_env(lib_a, seed), steps, seed, None, order, render_dir=da)
-    b = trace_chaotic(make_env(lib_b, seed, **kw), steps, seed, None, order, render_dir=db)
-    for d in (da, db):
+    d = tempfile.mkdtemp() if n_groups <= 4 else None
+    try:
+        return trace_chaotic(make_env(lib, seed, **kw), steps, seed, None, order, render_dir=d)
+    finally:
         if d is not None:
-            import shutil
             shutil.rmtree(d, ignore_errors=True)
+
+
+def play_chaotic(seed, lib_a, lib_b, steps=24, **kw):
+    a = chaotic_log(seed, lib_a, steps)
+    b = chaotic_log(seed, lib_b, steps, **kw)
     assert len(a) == len(b), "chaotic fuzz seed %d: %d vs %d records" % (seed, len(a), len(b))
     for ra, rb in zip(a, b):
         assert ra[0] == rb[0], "chaotic fuzz seed %d: %s vs %s" % (seed, ra[0], rb[0])

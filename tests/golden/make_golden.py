@@ -1,10 +1,12 @@
 #!/usr/bin/env python
 """Regenerate tests/golden/*.npz from the UNMODIFIED reference engine.
 
-Run in the build container (needs /root/reference):
+Run where the reference sources exist (oracle/Makefile, REF=<reference checkout>):
     make -C oracle ref && OMP_NUM_THREADS=1 python tests/golden/make_golden.py
 The reference is only deterministic single-threaded (SURVEY.md §0 fact 2), hence OMP_NUM_THREADS=1.
-Every scenario is recorded twice and must hash identically before it is written.
+Every scenario is recorded twice and must hash identically before it is written.  Last, the non-GPU suite runs with
+MAGENT_B200_RECORD_REFERENCE=1, which rewrites tests/golden/reference_results.npz: the results of the reference that
+the differential tests compare with (golden_common.check_reference_result).
 """
 import os
 import sys
@@ -32,3 +34,9 @@ if __name__ == "__main__":
     assert sorted(a) == sorted(b) and all(np.array_equal(a[k], b[k]) for k in a), "edge cases: reference not deterministic"
     np.savez_compressed(gc.EDGE_FILE, **a)
     print("edge_cases       %s" % sorted(a))
+    import subprocess
+    if os.path.exists(gc.RESULTS_FILE):
+        os.remove(gc.RESULTS_FILE)
+    subprocess.run([sys.executable, "-m", "pytest", "-q", "-m", "not gpu", os.path.dirname(HERE)],
+                   env=dict(os.environ, **{gc.RECORD_ENV: "1"}), check=True)
+    print("reference_results %6.1f KB" % (os.path.getsize(gc.RESULTS_FILE) / 1024))

@@ -1,6 +1,7 @@
 """Golden fixtures: traces recorded from the UNMODIFIED compiled reference (oracle/_ref, built from
 /root/reference by oracle/Makefile) with tests/golden/make_golden.py, committed as small .npz files so the
 parity suite has pinned vectors even where neither /root/reference nor oracle/_ref exists."""
+import hashlib
 import os
 
 import numpy as np
@@ -102,6 +103,67 @@ def record_edge_cases(lib, tmpdir):
     for name, data in files.items():
         out["self_kill_file_" + name] = np.frombuffer(data, dtype=np.uint8)
     return out
+
+
+
+# ------------------------------------------------------------------ recorded results of the reference, one per test case
+# Differential tests that used to run the compiled reference next to the library under test compare with these instead,
+# so they run where the reference cannot be built.  A result (nested dicts / lists / tuples of arrays, numbers, strings,
+# bytes) is stored as a fingerprint: the sha256 of every value that is compared exactly, and the rewards, which are
+# compared within REWARD_TOL as in compare_traces, in full.
+RESULTS_FILE = os.path.join(GOLDEN_DIR, "reference_results.npz")
+RECORD_ENV = "MAGENT_B200_RECORD_REFERENCE"     # =1: check_reference_result records the reference's result instead
+
+
+def fingerprint(result):
+    """(sha256 hex of the exactly compared part, float32 array of the rewards) of a nested result.  Rewards are the
+    'reward' entry of a run_trace record and the float32 arrays of a fuzz_common log record labelled '... reward ...'."""
+    h = hashlib.sha256()
+    rewards = []
+
+    def walk(x, reward=False):
+        if isinstance(x, dict):
+            h.update(b"{%d" % len(x))
+            for k in sorted(x, key=repr):
+                h.update(repr(k).encode())
+                walk(x[k], reward or k == "reward")
+        elif isinstance(x, (list, tuple)):
+            h.update(b"[%d" % len(x))
+            labelled = len(x) > 0 and isinstance(x[0], str) and " reward" in x[0]
+            for i, v in enumerate(x):
+                walk(v, reward or (labelled and i > 0 and getattr(v, "dtype", None) == np.float32))
+        elif isinstance(x, str):
+            h.update(b"s" + x.encode())
+        elif isinstance(x, bytes):
+            h.update(b"b%d:" % len(x) + x)
+        else:
+            a = np.asarray(x)
+            h.update(("%s%s" % (a.dtype, a.shape)).encode())
+            if reward:
+                rewards.append(a.astype(np.float32).ravel())
+            else:
+                h.update(np.ascontiguousarray(a).tobytes())
+    walk(result)
+    return h.hexdigest(), (np.concatenate(rewards) if rewards else np.zeros((0,), np.float32))
+
+
+def check_reference_result(key, run, lib):
+    """run(lib) must give the result run(oracle/_ref) gave when tests/golden/reference_results.npz was recorded
+    (tests/golden/make_golden.py)"""
+    if os.environ.get(RECORD_ENV) == "1":
+        a, b = fingerprint(run(pc.REF_LIB)), fingerprint(run(pc.REF_LIB))
+        assert a[0] == b[0] and np.array_equal(a[1], b[1]), key + ": reference not deterministic"
+        stored = dict(np.load(RESULTS_FILE)) if os.path.exists(RESULTS_FILE) else {}
+        stored[key + "/sha"] = np.frombuffer(bytes.fromhex(a[0]), dtype=np.uint8)
+        stored[key + "/reward"] = a[1]
+        np.savez_compressed(RESULTS_FILE, **stored)
+    z = np.load(RESULTS_FILE)
+    assert key + "/sha" in z.files, key + ": no recorded reference result"
+    sha, rewards = fingerprint(run(lib))
+    want = z[key + "/reward"]
+    assert rewards.shape == want.shape, "%s: %d rewards vs %d recorded from the reference" % (key, rewards.size, want.size)
+    np.testing.assert_allclose(rewards, want, rtol=0, atol=pc.REWARD_TOL, err_msg=key + " rewards")
+    assert sha == bytes(z[key + "/sha"]).hex(), key + ": differs from the result recorded from the reference"
 
 
 def check_edge_cases(lib, tmpdir, with_render=True):

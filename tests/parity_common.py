@@ -504,19 +504,24 @@ def compare_info_snapshots(a, b, what=""):
             np.testing.assert_array_equal(a[k], b[k], err_msg="%s %s" % (what, k))
 
 
-def play_and_compare_info(make, lib_a, lib_b, steps=6, seed=3):
-    ea, eb = make(lib_a), make(lib_b)
-    compare_info_snapshots(info_snapshot(ea, with_mean=False), info_snapshot(eb, with_mean=False), "before the first step")
+def info_log(make, lib, steps=6, seed=3):
+    """[(what, info_snapshot)] before the first step and after every step and clear_dead of a random-action game"""
+    env = make(lib)
+    log = [("before the first step", info_snapshot(env, with_mean=False))]
     rs = np.random.RandomState(seed)
     for t in range(steps):
-        for h in ea.get_handles():
-            act = rs.randint(0, ea.get_action_space(h)[0], size=ea.get_num(h)).astype(np.int32)
-            ea.set_action(h, act)
-            eb.set_action(h, act)
-        ea.step(); eb.step()
-        compare_info_snapshots(info_snapshot(ea), info_snapshot(eb), "after step %d" % t)
-        ea.clear_dead(); eb.clear_dead()
-        compare_info_snapshots(info_snapshot(ea), info_snapshot(eb), "after clear_dead %d" % t)
+        for h in env.get_handles():
+            env.set_action(h, rs.randint(0, env.get_action_space(h)[0], size=env.get_num(h)).astype(np.int32))
+        env.step()
+        log.append(("after step %d" % t, info_snapshot(env)))
+        env.clear_dead()
+        log.append(("after clear_dead %d" % t, info_snapshot(env)))
+    return log
+
+
+def play_and_compare_info(make, lib_a, lib_b, steps=6, seed=3):
+    for (what, a), (_, b) in zip(info_log(make, lib_a, steps, seed), info_log(make, lib_b, steps, seed)):
+        compare_info_snapshots(a, b, what)
 
 
 # ------------------------------------------------------------------ extensions: select_arena, event counters

@@ -75,10 +75,6 @@ def test_arena_batch_matches_single_arenas(emu):
 
 def test_mid_episode_add_agents_roundtrip(emu):
     """add_agents after stepping: device image -> host image -> mutate -> device image"""
-    ref = pc.REF_LIB if os.path.exists(pc.REF_LIB) else None
-    if ref is None:
-        pytest.skip("needs the compiled reference")
-
     def run(lib):
         env = pc.make_battle(lib, 30, 60, 2)
         hs = env.get_handles()
@@ -98,15 +94,11 @@ def test_mid_episode_add_agents_roundtrip(emu):
             out.append([env.get_agent_id(h).tolist() for h in hs])
             env.clear_dead()
         return out
-    assert run(ref) == run(emu)
+    gc.check_reference_result("mid_episode_add_agents", run, emu)
 
 
 def test_forty_rules(emu):
-    if not os.path.exists(pc.REF_LIB):
-        pytest.skip("needs the compiled reference")
-    want = pc.run_trace(pc.make_many_rules(pc.REF_LIB), 25, 5, keep_obs=True)
-    got = pc.run_trace(pc.make_many_rules(emu), 25, 5, keep_obs=True)
-    pc.compare_traces(want, got, "many rules")
+    gc.check_reference_result("forty_rules", lambda lib: pc.run_trace(pc.make_many_rules(lib), 25, 5, keep_obs=True), emu)
 
 
 def test_unsupported_rule_shapes_fail_loudly(emu):
@@ -124,12 +116,9 @@ def test_unsupported_rule_shapes_fail_loudly(emu):
 @pytest.mark.parametrize("seed", [13, 14, 15])
 def test_absorb_contention_matches_reference(emu, seed):
     """dense absorbers: several movers reach the same goal in one step; only the first in move order is absorbed"""
-    if not os.path.exists(pc.REF_LIB):
-        pytest.skip("needs the compiled reference")
     kw = dict(act_groups=[1], keep_obs=True, stop_on_done=False)
-    a = pc.run_trace(pc.make_arrange(pc.REF_LIB, 20, seed, n_goal=40, n_agent=200), 40, seed, **kw)
-    b = pc.run_trace(pc.make_arrange(emu, 20, seed, n_goal=40, n_agent=200), 40, seed, **kw)
-    pc.compare_traces(a, b, "absorb")
+    gc.check_reference_result("absorb_contention/%d" % seed,
+                              lambda lib: pc.run_trace(pc.make_arrange(lib, 20, seed, n_goal=40, n_agent=200), 40, seed, **kw), emu)
 
 
 def _render_episode(lib, tmpdir, scenario):

@@ -7,6 +7,7 @@ import os
 import pytest
 
 import fuzz_common as fz
+import golden_common as gc
 import parity_common as pc
 from test_emu_parity_cpu import emu  # noqa: F401  (fixture: builds tests/_emu on demand)
 
@@ -19,10 +20,9 @@ def test_emulated_engine_matches_checker_on_random_games(emu, seed):
     fz.play(seed, CHECKER, emu, steps=20)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs oracle/_ref (the compiled reference)")
 @pytest.mark.parametrize("seed", list(range(100, 116)) + list(range(1100, 1110)))
 def test_oracle_port_matches_reference_on_random_games(seed):
-    fz.play(seed, pc.REF_LIB, pc.PORT_LIB, steps=20)
+    gc.check_reference_result("fuzz/%d" % seed, lambda lib: fz.trace(seed, lib, steps=20), pc.PORT_LIB)
 
 
 @pytest.mark.parametrize("seed", list(range(200, 212)) + list(range(1200, 1206)))
@@ -44,10 +44,9 @@ def test_emulated_engine_matches_checker_on_banded_maps(emu, seed):
     fz.play(seed, CHECKER, emu, steps=15)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs oracle/_ref (the compiled reference)")
 @pytest.mark.parametrize("seed", list(range(100600, 100604)) + [200002])
 def test_oracle_port_matches_reference_on_banded_maps(seed):
-    fz.play(seed, pc.REF_LIB, pc.PORT_LIB, steps=15)
+    gc.check_reference_result("fuzz/%d" % seed, lambda lib: fz.trace(seed, lib, steps=15), pc.PORT_LIB)
 
 
 @pytest.mark.parametrize("seed", [101000, 101001, 101002, 201000])
@@ -68,10 +67,9 @@ def test_emulated_engine_matches_checker_with_a_chaotic_caller(emu, seed):
     fz.play_chaotic(seed, CHECKER, emu)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs oracle/_ref (the compiled reference)")
 @pytest.mark.parametrize("seed", list(range(43000, 43008)))
 def test_oracle_port_matches_reference_with_a_chaotic_caller(seed):
-    fz.play_chaotic(seed, pc.REF_LIB, pc.PORT_LIB)
+    gc.check_reference_result("fuzz_chaotic/%d" % seed, lambda lib: fz.chaotic_log(seed, lib), pc.PORT_LIB)
 
 
 @pytest.mark.parametrize("seed", list(range(60000, 60010)) + [115000, 115001])

@@ -141,8 +141,6 @@ def test_kat_shuffle_decides_mutual_kill(olib):
 @pytest.mark.parametrize("game", ["forest", "double_attack"])
 def test_port_matches_reference_beyond_golden(game):
     """the restatement's general rule evaluator (two free symbols in double_attack) vs the compiled reference"""
-    if not (os.path.exists(pc.REF_LIB) and os.path.exists(pc.PORT_LIB)):
-        pytest.skip("needs both oracle libraries")
     import magent_b200 as magent
 
     def make(lib):
@@ -153,18 +151,16 @@ def test_port_matches_reference_beyond_golden(game):
         env.add_agents(h[0], method="random", n=120)
         env.add_agents(h[1], method="random", n=60)
         return env
-    a = pc.run_trace(make(pc.REF_LIB), 60, 3, keep_obs=True)
-    b = pc.run_trace(make(pc.PORT_LIB), 60, 3, keep_obs=True)
-    pc.compare_traces(a, b, game)
+    gc.check_reference_result("port_beyond_golden/" + game, lambda lib: pc.run_trace(make(lib), 60, 3, keep_obs=True),
+                              pc.PORT_LIB)
 
 
-@pytest.mark.skipif(not os.path.exists(pc.REF_LIB), reason="needs oracle/_ref")
 @pytest.mark.parametrize("which", ["battle", "pursuit", "mixed", "arrange"])
 def test_port_serves_the_cold_info_getters_like_the_reference(which):
     """view2attack / attack_base / groups_info / walls_info / global_minimap / mean_info (GridWorld.cc:717-894)"""
     make = {"battle": lambda lib: pc.make_battle(lib, 30, 120, 1), "pursuit": lambda lib: pc.make_pursuit(lib, 40, 2),
             "mixed": lambda lib: pc.make_mixed(lib), "arrange": lambda lib: pc.make_arrange(lib)}[which]
-    pc.play_and_compare_info(make, pc.REF_LIB, pc.PORT_LIB)
+    gc.check_reference_result("cold_info/" + which, lambda lib: pc.info_log(make, lib), pc.PORT_LIB)
 
 
 def test_port_reproduces_the_golden_edge_cases():
@@ -174,17 +170,13 @@ def test_port_reproduces_the_golden_edge_cases():
     gc.check_edge_cases(pc.PORT_LIB, tempfile.mkdtemp())
 
 
-@pytest.mark.skipif(not os.path.exists(pc.REF_LIB), reason="needs oracle/_ref")
 @pytest.mark.parametrize("which", ["battle", "arrange", "turn", "food"])
 def test_port_writes_the_replay_dump_of_the_reference(tmp_path, which):
     """env_render: config.json + video_N.txt frames incl. attack events, render_window_info / attack_event
     (RenderGenerator.cc:56-185, GridWorld.cc:797-842)"""
+    import tempfile
     from test_emu_parity_cpu import _render_episode
     scen = {"battle": lambda lib: pc.make_battle(lib, 30, 200, 3), "arrange": lambda lib: pc.make_arrange(lib, 30, 12),
             "turn": lambda lib: pc.make_turn(lib, 30, 5), "food": lambda lib: pc.make_food(lib, 30, 3)}[which]
-    want = _render_episode(pc.REF_LIB, str(tmp_path / "ref"), scen)
-    got = _render_episode(pc.PORT_LIB, str(tmp_path / "port"), scen)
-    assert want[0].keys() == got[0].keys()
-    for name in want[0]:
-        assert want[0][name] == got[0][name], name
-    assert want[1] == got[1] and want[2] == got[2]
+    gc.check_reference_result("replay_dump/" + which, lambda lib: _render_episode(lib, tempfile.mkdtemp(dir=str(tmp_path)), scen),
+                              pc.PORT_LIB)
