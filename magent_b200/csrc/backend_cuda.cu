@@ -671,7 +671,10 @@ __global__ void __launch_bounds__(256) info_kernel(const EngineDev *gE, unsigned
         const long gi = (long)a * E.grp[g].cap + i;
         switch (kind) {
             case INFO_ID: ((int *)buf)[o] = s.id[gi]; break;
-            case INFO_POS: ((int2 *)buf)[o] = make_int2(s.x[gi], s.y[gi]); break;
+            case INFO_POS:                // int[n][2] needs only 4-byte alignment: one 8-byte store where the buffer allows it
+                if ((((size_t)buf) & 7) == 0) ((int2 *)buf)[o] = make_int2(s.x[gi], s.y[gi]);
+                else { ((int *)buf)[2 * (size_t)o] = s.x[gi]; ((int *)buf)[2 * (size_t)o + 1] = s.y[gi]; }
+                break;
             case INFO_ALIVE: ((unsigned char *)buf)[o] = (s.flags[gi] & FLAG_DEAD) ? 0 : 1; break;
             case INFO_REWARD: ((float *)buf)[o] = s.next_reward[gi] + E.hdr[a].grp_reward[g]; break;
             case INFO_HP: ((float *)buf)[o] = s.hp[gi]; break;
